@@ -57,6 +57,7 @@ def parse():
     ap.add_argument("--e2e-chunks", type=int, default=4, help="chunks of the window in the e2e leg (copy/compute overlap)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip latency / C4 / per-kernel roofline side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -127,6 +128,26 @@ def algorithmic_bytes(stats, n_feat: int) -> float:
     per residual pass, pose in/out + H + counters + visibility mask out."""
     return (49.0 * float(stats["sum_visible"]) + 65.0 * n_feat + 25.0 * float(stats["sum_in_image"]) +
             96 + 96 + 288 + 16 + n_feat)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, res: dict):
+    """The results of the timed path's last step as its caller receives them (sia_batch_fetch): relative poses T
+    [pairs, 3, 4] f64, visibility mask [pairs, features] f32 and the per-pair counters f64.  Above 64 MB in all, a fixed
+    seeded sample of the pairs is written, its indices in pairs.npy."""
+    B = len(res["T"])
+    arrays = {"T": res["T"], "visible": res["visible"].reshape(B, -1).astype(np.float32)}
+    arrays.update({k: res["stats"][k].astype(np.float64) for k in res["stats"].dtype.names})
+    per_pair = sum(a.nbytes for a in arrays.values()) / B + 8
+    if per_pair * B > DUMP_LIMIT_BYTES:
+        pairs = np.sort(np.random.default_rng(0).choice(B, int((DUMP_LIMIT_BYTES - 4096) // per_pair), replace=False))
+        arrays = {k: a[pairs] for k, a in arrays.items()}  # (4 KB left for the .npy headers)
+        arrays["pairs"] = pairs.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def make_inputs(seed: int, B: int, device: str):
@@ -516,6 +537,8 @@ def main():
     ms_dev = grp.max_over_ranks(ms_dev_local)
     res = ctx.sia_batch_fetch()
     stats = res["stats"]
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     alg_bytes = sum(algorithmic_bytes(stats[b], NFEAT) for b in range(B))
     kernel_ms = ms_dev / (K * passes)
 

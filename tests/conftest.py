@@ -22,6 +22,28 @@ def oracle():
     return binding
 
 
+_RECORDS = {}  # module -> test -> outputs of the compiled reference recorded in this session
+
+
+@pytest.fixture
+def reference(request):
+    """The outputs of the reference's own sources (oracle/_ref) for this test, replayed from tests/golden/reference/;
+    with SVO_RECORD_REFERENCE=DIR they are recorded from oracle/_ref into DIR instead (tests/reference_outputs.py)."""
+    from tests import reference_outputs
+
+    r = reference_outputs.Reference(request.node.module.__name__.rsplit(".", 1)[-1], request.node.name,
+                                    os.environ.get("SVO_RECORD_REFERENCE") or None)
+    yield r
+    r.finish(_RECORDS)
+
+
+def pytest_sessionfinish(session):
+    if _RECORDS:
+        from tests import reference_outputs
+
+        reference_outputs.write(os.environ["SVO_RECORD_REFERENCE"], _RECORDS)
+
+
 @pytest.fixture(scope="session")
 def ctx():
     """A CUDA context of the product library; fails loudly when there is no GPU."""

@@ -12,11 +12,6 @@ from rpg_svo_b200 import synth
 CAMERAS = ["atan", "pinhole_radtan"]
 
 
-def _need_ref(oracle):
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
-
-
 @pytest.mark.parametrize("kind", CAMERAS)
 def test_camera_functions_oracle_vs_numpy(oracle, kind):
     cam = synth.reference_param_camera(kind)
@@ -35,14 +30,13 @@ def test_camera_functions_oracle_vs_numpy(oracle, kind):
 
 
 @pytest.mark.parametrize("kind", CAMERAS)
-def test_oracle_sparse_img_align_distorted_equals_reference_source_compiled_here(oracle, kind):
+def test_oracle_sparse_img_align_distorted_equals_reference_source_compiled_here(oracle, kind, reference):
     """The reference's SparseImgAlign (oracle/_ref) over the shim's vk::ATANCamera / distorted vk::PinholeCamera vs the
     oracle: same visibility, same pose."""
-    _need_ref(oracle)
     cam = synth.reference_param_camera(kind)
     p = synth.make_frame_pair(61, n_feat=200, cam=cam)
-    r = oracle.ref_sparse_img_align(p["ref_pyr"][0], p["cur_pyr"][0], p["n_levels"], cam, p["T_ref_w"], p["T_ref_w"], p["px"],
-                                    p["f"], p["pos"], p["has_point"], 4, 0)
+    r = reference.ref_sparse_img_align(p["ref_pyr"][0], p["cur_pyr"][0], p["n_levels"], cam, p["T_ref_w"], p["T_ref_w"], p["px"],
+                                       p["f"], p["pos"], p["has_point"], 4, 0)
     o = oracle.sparse_img_align(p["ref_pyr"], p["cur_pyr"], cam, synth.se3_identity(), p["px"], p["f"], p["pos"],
                                 p["has_point"], p["ref_pos"], 4, 0)
     assert r["n_tracked"] == o["n_tracked"] > 100
@@ -52,17 +46,16 @@ def test_oracle_sparse_img_align_distorted_equals_reference_source_compiled_here
 
 
 @pytest.mark.parametrize("kind", CAMERAS)
-def test_oracle_matcher_distorted_equals_reference_source_compiled_here(oracle, kind):
-    _need_ref(oracle)
+def test_oracle_matcher_distorted_equals_reference_source_compiled_here(oracle, kind, reference):
     cam = synth.reference_param_camera(kind)
     c = synth.make_match_case(23, 60, cam=cam)
     T_cur_ref = synth.se3_mul(c["T_cur_w"], synth.se3_inv(c["T_ref_w"]))
     ref_pos = synth.se3_inv(c["T_ref_w"])[:, 3]
     n_ok = 0
     for i in range(c["M"]):
-        r = oracle.ref_matcher(0, c["ref_pyr"][0], c["cur_pyr"][0], c["n_levels"], cam, c["T_ref_w"], c["T_cur_w"],
-                               c["ref_px"][i], c["ref_f"][i], int(c["ref_level"][i]), int(c["ftr_type"][i]), c["ref_grad"][i],
-                               c["point_pos"][i], px_cur=c["px_cur"][i], n_pyr_levels=3)
+        r = reference.ref_matcher(0, c["ref_pyr"][0], c["cur_pyr"][0], c["n_levels"], cam, c["T_ref_w"], c["T_cur_w"],
+                                  c["ref_px"][i], c["ref_f"][i], int(c["ref_level"][i]), int(c["ftr_type"][i]), c["ref_grad"][i],
+                                  c["point_pos"][i], px_cur=c["px_cur"][i], n_pyr_levels=3)
         depth = np.linalg.norm(c["point_pos"][i] - ref_pos)
         o = oracle.find_match_direct(c["ref_pyr"], c["cur_pyr"], cam, T_cur_ref, c["ref_px"][i], c["ref_f"][i],
                                      int(c["ref_level"][i]), int(c["ftr_type"][i]), c["ref_grad"][i], depth, 2, 10, c["px_cur"][i])

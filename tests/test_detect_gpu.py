@@ -46,14 +46,12 @@ def test_fast_detect_noise_image_and_options(ctx, oracle):
     fr.destroy()
 
 
-def test_fast_detect_vs_compiled_reference(ctx, oracle):
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref not present on this box")
+def test_fast_detect_vs_compiled_reference(ctx, oracle, reference):
     d = synth.make_two_view(7, n_levels=5)
     fr = ctx.frame(d["ref_pyr"])
     occ = (np.random.default_rng(2).uniform(size=26 * 16) < 0.3).astype(np.uint8)
     g = ctx.fast_detect(fr, 30, 3, 20.0, occ)
-    r = oracle.ref_fast_detect(d["ref_pyr"][0], 5, 3, 30, 20.0, occ)
+    r = reference.ref_fast_detect(d["ref_pyr"][0], 5, 3, 30, 20.0, occ)
     _same(g, r)
     assert len(r["x"]) > 100
     fr.destroy()

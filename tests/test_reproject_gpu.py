@@ -41,11 +41,9 @@ def test_reproject_map_matches_oracle(ctx, oracle, seed, kw):
     assert g["n_speculative"] >= g["n_trials"] - (c["pt_type"] == 0).sum()   # the device aligned more than the policy used
 
 
-def test_reproject_map_vs_compiled_reference(ctx, oracle):
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref not present on this box")
+def test_reproject_map_vs_compiled_reference(ctx, oracle, reference):
     c = synth.make_map_case(9, n_kfs=10, n_points=800)
-    g, r = _run_gpu(ctx, c), oracle.ref_reproject_map(c)
+    g, r = _run_gpu(ctx, c), reference.ref_reproject_map(c)
     _same(g, r)
     assert np.array_equal(np.minimum(g["pt_action"], 2), np.minimum(r["pt_action"], 2))
     assert g["n_matches"] == c["options"]["max_fts"] + 1                     # the maxFts stop was reached
